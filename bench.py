@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the shading pass hot path (BASELINE.json: Msamples/s at 1920x1080x64spp).
 
-  python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C3|C2|C4|C1|mini]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload C3|C2|C4|C1|mini] [--dump-outputs DIR]
 
 A "step" is one pass of the shading megakernel over one frame of a synthetic scene. The default workload is BASELINE config 3, the
 one the metric is quoted on: the Bistro-like city (2.8 M triangles) at 1920x1080, 8 quad lights, 64 spp, diffuse+specular MIS with the
@@ -234,6 +234,13 @@ def run_b200(args):
 			dist.all_reduce(t, op=dist.ReduceOp.MAX)
 		return float(t.item())
 
+	def frame_of_this_rank():
+		if exchange is None:
+			return out.cpu().numpy()
+		host = np.empty((height, width, 4), dtype=np.float32)
+		assert lib.vkr_frame_exchange_download(C.byref(exchange), C.byref(frame.device), host.ctypes.data) == 0
+		return host
+
 	# kernel-only timing (per launch, CUDA events inside the library on the launching stream)
 	p.timing_enabled = 1
 	if world > 1:
@@ -247,6 +254,8 @@ def run_b200(args):
 	total_ms = timed(step_device, args.steps, 0)
 	launches = (int(p.kernel_launches) - launches_before) * world * (3 if exchange is not None else 1)   # every rank: the shading kernel (+ signal and wait of the exchange)
 	clocks = sampler.stop() if rank == 0 else None
+	if args.dump_outputs and rank == 0:
+		dump_outputs(args.dump_outputs, {"frame": frame_of_this_rank()})
 	# one more step to read the kernel's own duration on every rank
 	flush.zero_(); step_device(); lib.vkr_shading_pass_wait(C.byref(p), C.byref(frame.device))
 	if exchange is not None:
@@ -261,15 +270,9 @@ def run_b200(args):
 	value = samples / (ms_per_step * 1e-3) / 1e6
 
 	# --- the frame every rank holds now against a single-GPU render of the same frame (rank 0 renders it alone)
-	def frame_bytes_of_this_rank():
-		if exchange is None:
-			return out.cpu().numpy().tobytes()
-		host = np.empty((height, width, 4), dtype=np.float32)
-		assert lib.vkr_frame_exchange_download(C.byref(exchange), C.byref(frame.device), host.ctypes.data) == 0
-		return host.tobytes()
 	frame_check = None
 	if world > 1:
-		mine = hashlib.sha256(frame_bytes_of_this_rank()).hexdigest()
+		mine = hashlib.sha256(frame_of_this_rank().tobytes()).hexdigest()
 		single = None
 		if rank == 0:
 			whole = frame.create_pass(width, height)
@@ -384,6 +387,23 @@ def run_b200(args):
 		sys.exit(3)
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(directory, arrays):
+	"""Writes each array as <directory>/<name>.npy (float32) so that two builds can be compared output for output. An array over its share of
+	DUMP_LIMIT_BYTES is cut to a fixed, seeded sample of its rows (the same rows for the same shape), in ascending row order."""
+	os.makedirs(directory, exist_ok=True)
+	share = DUMP_LIMIT_BYTES // len(arrays)
+	for name, a in arrays.items():
+		a = np.ascontiguousarray(a, dtype=np.float32)
+		if a.nbytes > share:
+			keep = share // (a.nbytes // a.shape[0])
+			a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+			log("[bench] %s: %d of its rows written (fixed sample, seed 0)" % (name, keep))
+		np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def host_threads():
 	"""All host threads, whatever the launcher put into OMP_NUM_THREADS (torchrun sets it to 1)."""
 	try:
@@ -392,12 +412,13 @@ def host_threads():
 		return os.cpu_count() or 1
 
 
-def cpu_baseline(args, info, w, constants, band_stride_tiles=None, visibility=None, repeat=1):
+def cpu_baseline(args, info, w, constants, band_stride_tiles=None, visibility=None, repeat=1, shaded_rows=None):
 	"""Times the reference's path on the host cores on a bounded sample: 8-row bands spread over the frame, full light count and spp.
 	kind "reference": the reference's own shader sources compiled for the CPU (oracle/_ref/libref_shader.so, built by
 	oracle/build_ref.py where /root/reference exists and shipped prebuilt; it starts from the visibility buffer like the
 	shader does, i.e. it includes get_shading_data). kind "port": the C restatement (oracle/) when that library or this
-	configuration is not available. Both use OpenMP over 64-pixel pieces of rows with all host threads."""
+	configuration is not available. Both use OpenMP over 64-pixel pieces of rows with all host threads. shaded_rows: a list that receives the rows
+	of the sample as shaded by the last repetition, float32 [rows, width, 4]."""
 	from tests import harness as H
 	width, height, lights, spp, rays = w["width"], w["height"], w["lights"], w["spp"], w.get("rays", 1)
 	oi = H.OracleInputs(info)
@@ -422,7 +443,7 @@ def cpu_baseline(args, info, w, constants, band_stride_tiles=None, visibility=No
 				visibility = oi.visibility(width, height, constants)
 			t0 = time.time()
 			R.set_threads(host_threads())
-			R.shade(ref_cfg["entry"], width, height, ref_cfg, constants, visibility, oi.vks, oi.material_params, oi.noise, oi.ltc0, oi.ltc1, oi.shadow_tris, band_height=8, band_stride=band_stride)
+			frame = R.shade(ref_cfg["entry"], width, height, ref_cfg, constants, visibility, oi.vks, oi.material_params, oi.noise, oi.ltc0, oi.ltc1, oi.shadow_tris, band_height=8, band_stride=band_stride)
 			seconds = R.last_shade_seconds(); cores = R.thread_count(); kind = "reference"
 			what = "the reference's shader sources (shading_pass.frag.glsl + includes) compiled as C++ with g++ -O2, fp32, OpenMP, ray queries on a CPU BVH"
 			log("[bench] cpu reference shader: %d rows in %.2f s on %d threads (+ %.1f s BVH build)" % (rows, seconds, cores, time.time() - t0 - seconds))
@@ -432,11 +453,13 @@ def cpu_baseline(args, info, w, constants, band_stride_tiles=None, visibility=No
 				row_begin=0, row_end=0, band_height=8, band_stride=band_stride)
 			gbuffer = oi.gbuffer(width, height, constants, visibility if visibility is not None else oi.visibility(width, height, constants))
 			H.oracle.set_threads(host_threads())
-			_, n_rays = H.oracle.shade(cfg, constants, gbuffer, oi.noise, oi.ltc0, oi.ltc1, oi.shadow_tris)
+			frame, n_rays = H.oracle.shade(cfg, constants, gbuffer, oi.noise, oi.ltc0, oi.ltc1, oi.shadow_tris)
 			seconds = H.oracle.last_shade_seconds(); cores = H.oracle.thread_count(); kind = "port"
 			what = "scalar fp32 C oracle, OpenMP"
 			log("[bench] cpu oracle: %d rows in %.2f s on %d threads (+ %.1f s BVH build), %d shadow rays" % (rows, seconds, cores, time.time() - t0 - seconds, n_rays))
 		seconds_all.append(seconds)
+	if shaded_rows is not None:
+		shaded_rows.append(frame[[y for y in range(height) if y % band_stride < 8]])
 	seconds = float(np.mean(seconds_all))
 	value = rows * width * spp / seconds / 1e6
 	return {"value": round(value, 4), "unit": "Msamples/s", "cores": cores, "kind": kind,
@@ -472,10 +495,13 @@ def run_reference(args):
 	stride = args.cpu_band_stride
 	while stride < 64 and sum(1 for y in range(height) if y % (8 * stride) < 8) > rows_allowed:
 		stride *= 2
+	shaded_rows = []
 	for i in range(args.warmup + args.steps):
-		r = cpu_baseline(args, info, w, constants, band_stride_tiles=stride, visibility=vis)
+		r = cpu_baseline(args, info, w, constants, band_stride_tiles=stride, visibility=vis, shaded_rows=shaded_rows)
 		if i >= args.warmup:
 			values.append(r)
+	if args.dump_outputs:
+		dump_outputs(args.dump_outputs, {"frame": shaded_rows[-1]})
 	seconds = sum(r["seconds"] for r in values)
 	value = float(np.mean([r["value"] for r in values]))
 	base = values[-1]
@@ -514,7 +540,11 @@ def main():
 	ap.add_argument("--no-counters", action="store_true", help="skip the extra untimed launch of the counters edition of the kernel")
 	ap.add_argument("--cpu-port", action="store_true", help="time the C restatement (oracle/) on the CPU legs even if the compiled reference shader is available")
 	ap.add_argument("--cpu-band-stride", type=int, default=4, help="the CPU sample takes one 8-row band every this many tile rows")
+	ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step shaded to DIR/frame.npy (float32 [rows, width, 4]: the whole frame; "
+		"with --impl reference the rows of its sample; above 64 MiB a fixed, seeded sample of those rows)")
 	args = ap.parse_args()
+	if args.steps < 1:
+		ap.error("--steps must be at least 1")
 	if args.warmup < 3:
 		log("[bench] note: the timing rules ask for at least 3 warm-up steps (got %d)" % args.warmup)
 	if args.impl == "reference":

@@ -273,16 +273,16 @@ def build_host():
 
 def build_c_host():
 	"""tests/c_host/route_b.c: a plain C host that loads a data set with the reference's UNCHANGED loaders (over shim/), hands their buffers to
-	libvkr_b200.so and renders a frame through the C-ABI (INTEGRATION.md, Routes B and A) -> tests/build/route_b. Needs /root/reference and the built library."""
+	libvkr_b200.so and renders a frame through the C-ABI (INTEGRATION.md, Routes B and A) -> oracle/_ref/route_b, next to the other binaries built from
+	the reference's sources. Needs the reference's sources and the built library."""
 	ref_src = "/root/reference/src"
 	root = os.path.dirname(HERE)
 	package = os.path.join(root, "vulkan_renderer_b200")
 	if not os.path.isdir(ref_src) or not os.path.exists(os.path.join(package, "libvkr_b200.so")):
 		return None
 	shim = os.path.join(root, "shim")
-	out_dir = os.path.join(root, "tests", "build")
-	os.makedirs(out_dir, exist_ok=True)
-	binary = os.path.join(out_dir, "route_b")
+	os.makedirs(OUT, exist_ok=True)
+	binary = os.path.join(OUT, "route_b")
 	sources = [os.path.join(ref_src, n) for n in ("scene.c", "textures.c", "ltc_table.c", "noise_table.c")]
 	cmd = ["/usr/bin/gcc", "-O2", "-std=gnu11", "-w", "-ffp-contract=off", "-I", shim, "-I", ref_src, "-I", os.path.join(root, "include"),
 		os.path.join(root, "tests", "c_host", "route_b.c"), os.path.join(shim, "vkr_shim.c")] + sources + ["-L", package, "-l:libvkr_b200.so", "-Wl,-rpath,$ORIGIN/../../vulkan_renderer_b200", "-lm", "-o", binary]

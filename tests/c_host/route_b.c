@@ -5,7 +5,7 @@
  * buffers, images and the triangle soup of the acceleration structure build are handed to libvkr_b200.so (vkr_scene_from_buffers,
  * vkr_ltc_table_from_images, vkr_noise_table_from_image). Route A from there on: the frame-side C-ABI renders one frame (visibility pass, G-buffer
  * pass, shading pass) and the program writes it as raw float32 RGBA. No Python, no ctypes: this is what a maintainer of the reference would link.
- * Built by oracle/build_ref.py (needs /root/reference) into tests/build/route_b; tests/test_gpu_zzzz_c_host.py runs it on the GPU box and compares the
+ * Built by oracle/build_ref.py (needs the reference's sources) into oracle/_ref/route_b; tests/test_gpu_zzzz_c_host.py runs it on the GPU box and compares the
  * frame with the oracle.
  *
  *   route_b <scene.vks> <texture dir> <quicksave> <ltc dir> <width> <height> <sample count> <out.f32>

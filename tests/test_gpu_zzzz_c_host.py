@@ -1,6 +1,6 @@
 """Boundaries B1 + B2 with a plain C host (SURVEY 8b, INTEGRATION.md): tests/c_host/route_b.c loads a data set with the reference's UNCHANGED loaders
 (compiled from /root/reference against shim/), hands their buffers and images to libvkr_b200.so and renders a frame through the C-ABI. The frame
-must equal the oracle's, bit for bit. The binary is built by oracle/build_ref.py where /root/reference exists and travels prebuilt."""
+must equal the oracle's, bit for bit. build() compiles the binary into oracle/_ref/route_b where the reference's sources are present; it travels prebuilt."""
 import os
 import subprocess
 
@@ -12,8 +12,8 @@ from tests.ref_frames import host_constants
 from vulkan_renderer_b200 import api
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BINARY = os.path.join(ROOT, "tests", "build", "route_b")
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not os.path.exists(BINARY), reason="tests/build/route_b not built (needs /root/reference)")]
+BINARY = os.path.join(ROOT, "oracle", "_ref", "route_b")
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not os.path.exists(BINARY), reason="oracle/_ref/route_b not built (needs the reference's loader sources)")]
 
 
 @pytest.mark.parametrize("name,width,height,spp", [("cornell", 128, 96, 2), ("mini_city", 160, 96, 2)])

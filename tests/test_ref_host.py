@@ -1,137 +1,113 @@
 """Boundary B1 (SURVEY 8b): the reference's UNCHANGED loader and host-maths sources, compiled against shim/ into
 oracle/_ref/libref_host.so, load the synthetic datasets; what they upload through the shim must equal, byte for byte,
 what libvkr_b200.so's own loaders produce. Also pins the host maths (update_polygonal_light, camera matrices,
-matrix_inverse) of vkr_host.cpp against the reference's code. Skipped where the reference-derived binary is absent."""
+matrix_inverse) of vkr_host.cpp against the reference's code. What the reference's code produced is stored in
+tests/golden/ref_host.json (tools/make_ref_golden.py host): small values as they are, large buffers as sha256 digests."""
 import ctypes as C
+import json
 import os
 
 import numpy as np
 import pytest
 
 from tests import harness as H
+from tests.ref_frames import camera_trials, digest, host_constants, light_trials
 from vulkan_renderer_b200 import api
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_HOST = os.path.join(ROOT, "oracle", "_ref", "libref_host.so")
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_HOST), reason="oracle/_ref/libref_host.so not built (needs /root/reference)")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_host.json")
 
 
 @pytest.fixture(scope="module")
 def ref():
-	lib = C.CDLL(REF_HOST)
-	lib.ref_probe_material_name.restype = C.c_char_p
-	lib.ref_probe_material_name.argtypes = [C.c_uint64]
-	lib.ref_probe_sizes.restype = C.c_uint32
-	return lib
+	with open(GOLDEN) as f:
+		return json.load(f)
 
 
 def test_struct_sizes(ref):
-	assert [ref.ref_probe_sizes(i) for i in range(5)] == [C.sizeof(api.Camera), C.sizeof(api.PolygonalLight), 88, 160, C.sizeof(api.LtcConstants)]
+	assert ref["struct_sizes"] == [C.sizeof(api.Camera), C.sizeof(api.PolygonalLight), 88, 160, C.sizeof(api.LtcConstants)]
 
 
 @pytest.mark.parametrize("name", ["cornell", "mini_city"])
 def test_reference_load_scene_through_the_shim_equals_our_loader(ref, name):
+	g = ref["scenes"][name]
 	info = H.dataset(name)
-	tri = C.c_uint64(); mat = C.c_uint64(); fs = (C.c_float * 6)(); pos = C.c_void_p(); nuv = C.c_void_p(); mi = C.c_void_p(); soup = C.POINTER(C.c_float)(); ntri = C.c_uint64()
-	assert ref.ref_probe_load_scene(info["vks"].encode(), info["textures"].encode(), C.byref(tri), C.byref(mat), fs, C.byref(pos), C.byref(nuv), C.byref(mi), C.byref(soup), C.byref(ntri)) == 0
-	n = tri.value
+	assert digest(open(info["vks"], "rb").read()) == g["vks_sha256"], "the synthetic scene generator drifted: regenerate with tools/make_ref_golden.py"
+	n = g["triangle_count"]
 	lib = api.load_library()
 	scene = api.Scene()
 	assert lib.vkr_load_scene(C.byref(scene), None, info["vks"].encode(), info["textures"].encode(), 1) == 0
-	assert n == scene.triangle_count == info["triangle_count"] and mat.value == scene.material_count
-	assert list(fs) == list(scene.dequantization_factor) + list(scene.dequantization_summand)
+	assert n == scene.triangle_count == info["triangle_count"] and g["material_count"] == scene.material_count
+	assert g["dequantization"] == list(scene.dequantization_factor) + list(scene.dequantization_summand)
 	vks = H.read_vks(info["vks"])
-	assert np.array_equal(np.ctypeslib.as_array(C.cast(pos, C.POINTER(C.c_uint32)), (3 * n, 2)), vks["positions"])
-	assert np.array_equal(np.ctypeslib.as_array(C.cast(nuv, C.POINTER(C.c_uint16)), (3 * n, 4)), vks["normals_uv"])
-	assert np.array_equal(np.ctypeslib.as_array(C.cast(mi, C.POINTER(C.c_uint8)), (n,)), vks["material_indices"])
+	assert digest(vks["positions"]) == g["positions_sha256"]
+	assert digest(vks["normals_uv"]) == g["normals_uv_sha256"]
+	assert digest(vks["material_indices"]) == g["material_indices_sha256"]
 	# the triangle soup handed to vkCmdBuildAccelerationStructuresKHR (scene.c:175-209) == what our shadow BVH is built from
-	assert ntri.value == n
-	ref_soup = np.ctypeslib.as_array(soup, (n, 9))
-	ours = H.oracle.dequantize_for_bvh(vks["positions"], vks["factor"], vks["summand"])
-	assert np.array_equal(ref_soup.view(np.uint32), ours.view(np.uint32))
+	assert g["soup_triangle_count"] == n
+	assert digest(H.oracle.dequantize_for_bvh(vks["positions"], vks["factor"], vks["summand"]).astype(np.float32)) == g["soup_sha256"]
 	# materials: names and the texel our constant-material model takes from each *.vkt
 	mp = np.ctypeslib.as_array(scene.material_params, (scene.material_count, 8))
-	for m in range(mat.value):
-		assert ref.ref_probe_material_name(m) == scene.material_names[m]
-		texel = (C.c_uint16 * 8)()
+	for m in range(g["material_count"]):
+		assert g["material_names"][m].encode() == scene.material_names[m]
 		for t, cols in ((0, (0, 1, 2)), (1, (None, 3, 4)), (2, (5, 6, None))):
-			assert ref.ref_probe_material_texel(C.c_uint64(m), t, texel) == 97
-			half = np.frombuffer(bytes(texel), dtype=np.float16)[:4].astype(np.float32)
+			texel = g["material_texels"][m][t]
+			assert texel["format"] == 97
 			for k, col in enumerate(cols):
 				if col is not None:
-					assert half[k] == mp[m, col]
-	ref.ref_probe_destroy_scene(); lib.vkr_destroy_scene(C.byref(scene), None)
+					assert texel["rgba"][k] == mp[m, col]
+	lib.vkr_destroy_scene(C.byref(scene), None)
 
 
 def test_reference_ltc_and_noise_tables_through_the_shim(ref):
 	info = H.dataset("cornell")
 	lib = api.load_library()
-	res = C.c_uint32(); t0 = C.c_void_p(); t1 = C.c_void_p(); consts = (C.c_float * 8)()
-	assert ref.ref_probe_load_ltc(info["ltc"].encode(), 51, C.byref(res), C.byref(t0), C.byref(t1), consts) == 0
+	g = ref["ltc"]
 	ltc = api.LtcTable()
 	assert lib.vkr_load_ltc_table(C.byref(ltc), None, info["ltc"].encode(), 51) == 0
-	r = res.value
+	r = g["resolution"]
 	assert r == ltc.roughness_count == 64
-	assert np.array_equal(np.ctypeslib.as_array(C.cast(t0, C.POINTER(C.c_uint16)), (51, r, r, 4)), np.ctypeslib.as_array(ltc.h_table0, (51, r, r, 4)))
-	assert np.array_equal(np.ctypeslib.as_array(C.cast(t1, C.POINTER(C.c_uint16)), (51, r, r, 2)), np.ctypeslib.as_array(ltc.h_table1, (51, r, r, 2)))
-	assert bytes(consts) == bytes(ltc.constants)
-	ref.ref_probe_destroy_ltc(); lib.vkr_destroy_ltc_table(C.byref(ltc), None)
+	assert digest(np.ctypeslib.as_array(ltc.h_table0, (51, r, r, 4))) == g["table0_sha256"]
+	assert digest(np.ctypeslib.as_array(ltc.h_table1, (51, r, r, 2))) == g["table1_sha256"]
+	assert bytes(ltc.constants).hex() == g["constants"]
+	lib.vkr_destroy_ltc_table(C.byref(ltc), None)
 	for animate in (0, 1):
-		data = C.c_void_p(); mr = (C.c_uint32 * 7)()
-		assert ref.ref_probe_load_noise(256, 256, 64, 0, C.byref(data), mr, animate) == 0
+		g = ref["noise"][animate]
 		noise = api.NoiseTable()
 		assert lib.vkr_load_noise_table(C.byref(noise), None, 256, 256, 64, api.NOISE_WHITE) == 0
-		assert np.array_equal(np.ctypeslib.as_array(C.cast(data, C.POINTER(C.c_uint16)), (64 * 256 * 256 * 4,)), np.ctypeslib.as_array(noise.h_noise, (64 * 256 * 256 * 4,)))
+		assert digest(np.ctypeslib.as_array(noise.h_noise, (64 * 256 * 256 * 4,))) == g["data_sha256"]
 		masks = (C.c_uint32 * 2)(); layer = C.c_uint32(); rnd = (C.c_uint32 * 4)()
 		lib.vkr_set_noise_constants(masks, C.byref(layer), rnd, C.byref(noise), animate)
-		assert list(mr) == list(masks) + [layer.value] + list(rnd)
-		ref.ref_probe_destroy_noise(); lib.vkr_destroy_noise_table(C.byref(noise), None)
+		assert g["masks"] == list(masks) + [layer.value] + list(rnd)
+		lib.vkr_destroy_noise_table(C.byref(noise), None)
 
 
 def test_host_maths_matches_the_reference_bit_for_bit(ref):
+	"""Per trial, the digest of what the reference's update_polygonal_light left (the first 160 bytes of the light, world-space vertices, fan areas)
+	and of its world-to-projection matrix."""
 	lib = api.load_library()
 	rng = np.random.default_rng(11)
-	for trial in range(200):
-		n = int(rng.integers(3, 8))
-		light = api.PolygonalLight()
-		for i in range(3):
-			light.rotation_angles[i] = rng.uniform(-3.2, 3.2); light.translation[i] = rng.uniform(-50, 50); light.radiant_flux[i] = rng.uniform(0.1, 100)
-		light.scaling_x = rng.uniform(0.1, 5); light.scaling_y = rng.uniform(0.1, 5)
-		ang = np.sort(rng.uniform(0, 2 * np.pi, n))
-		if trial % 2: ang = ang[::-1]                       # both windings (the plane gets flipped for clockwise polygons)
-		vp = np.zeros((n, 4), dtype=np.float32); vp[:, 0] = np.cos(ang) * rng.uniform(0.5, 1.5); vp[:, 1] = np.sin(ang) * rng.uniform(0.5, 1.5)
-		ref_bytes = (C.c_uint8 * 160).from_buffer_copy(bytes(light)[:160])
-		vw_ref = np.zeros((n, 4), dtype=np.float32); fa_ref = np.zeros((n - 2, 4), dtype=np.float32)
-		ref.ref_probe_update_light(ref_bytes, n, vp.ctypes.data, vw_ref.ctypes.data, fa_ref.ctypes.data)
+	for trial, (n, light, vp) in enumerate(light_trials(rng)):
 		lib.vkr_set_polygonal_light_vertex_count(C.byref(light), n)
 		C.memmove(light.vertices_plane_space, vp.ctypes.data, vp.nbytes)
 		lib.vkr_update_polygonal_light(C.byref(light))
-		ours = bytearray(bytes(light)[:160]); theirs = bytearray(bytes(ref_bytes))
-		assert ours == theirs, trial
-		assert np.array_equal(np.ctypeslib.as_array(light.vertices_world_space, (n, 4)).view(np.uint32), vw_ref.view(np.uint32))
-		assert np.array_equal(np.ctypeslib.as_array(light.fan_areas, (n - 2, 4)).view(np.uint32), fa_ref.view(np.uint32))
+		ours = digest(bytes(light)[:160], np.ctypeslib.as_array(light.vertices_world_space, (n, 4)), np.ctypeslib.as_array(light.fan_areas, (n - 2, 4)))
+		assert ours == ref["lights_sha256"][trial], trial
 		lib.vkr_destroy_polygonal_light(C.byref(light))
-	for trial in range(200):
-		cam = api.Camera()
-		for i in range(3): cam.position_world_space[i] = rng.uniform(-100, 100)
-		cam.rotation_z = rng.uniform(-7, 7); cam.rotation_x = rng.uniform(0, 3.14); cam.vertical_fov = rng.uniform(0.3, 2.0); cam.near_plane = 0.05; cam.far_plane = 1000.0
-		aspect = np.float32(rng.uniform(0.5, 2.5))
-		a = (C.c_float * 16)(); b = (C.c_float * 16)()
-		ref.ref_probe_world_to_projection(C.byref(cam), C.c_float(aspect), a)
+	for trial, (cam, aspect) in enumerate(camera_trials(rng)):
+		b = (C.c_float * 16)()
 		lib.vkr_get_world_to_projection_space(b, C.byref(cam), C.c_float(aspect))
-		assert bytes(a) == bytes(b), trial
+		assert digest(bytes(b)) == ref["cameras_sha256"][trial], trial
 
 
 def test_constant_block_pixel_to_ray_uses_the_reference_inverse(ref):
 	"""vkr_write_constants inverts the projection with the reference's cofactor expansion (math_utilities.h:24-46)."""
 	info = H.dataset("mini_city")
-	from tests.ref_frames import host_constants
 	cb = host_constants(info, 320, 200, 3)
 	w2p = np.frombuffer(cb[32:96], dtype=np.float32).reshape(4, 4).copy()
 	w2p[:3, 3] = 0.0
-	inv = (C.c_float * 16)()
-	ref.ref_probe_matrix_inverse(w2p.ctypes.data, inv)
-	inv = np.frombuffer(bytes(inv), dtype=np.float32).reshape(4, 4)
+	assert w2p.tobytes().hex() == ref["inverse"]["input"], "the constant block drifted: regenerate with tools/make_ref_golden.py"
+	inv = np.frombuffer(bytes.fromhex(ref["inverse"]["output"]), dtype=np.float32).reshape(4, 4)
 	vt = np.array([np.float32(2.0) / np.float32(320), np.float32(2.0) / np.float32(200)], dtype=np.float32)
 	p2p = np.array([[vt[0], 0, np.float32(0.5) * vt[0] - np.float32(1)], [0, vt[1], np.float32(0.5) * vt[1] - np.float32(1)], [0, 0, 1], [0, 0, 1]], dtype=np.float32)
 	expect = np.zeros((3, 4), dtype=np.float32)
@@ -148,12 +124,11 @@ def test_constant_block_pixel_to_ray_uses_the_reference_inverse(ref):
 @pytest.mark.parametrize("name,lights,width,height", [("cornell", 1, 128, 96), ("mini_city", 3, 320, 192), ("mini_room", 32, 64, 48)])
 def test_constant_block_equals_the_reference_host_code(ref, name, lights, width, height):
 	"""vkr_write_constants against quick_load + write_constants of the reference (restated over its own structs and functions in oracle/ref_host_probe.c)."""
-	from tests.ref_frames import host_constants
 	info = H.dataset(name)
 	ours = host_constants(info, width, height, lights, sample_count=4)
-	theirs = H.reference_constants(info, width, height, lights, sample_count=4)
-	assert len(ours) == len(theirs)
-	assert ours == theirs
+	theirs = ref["constants"]["%s_%d_%dx%d" % (name, lights, width, height)]
+	assert len(ours) == theirs["size"]
+	assert digest(ours) == theirs["sha256"]
 
 
 def test_noise_blob_files_are_read_as_the_reference_lays_them_out(tmp_path, monkeypatch):

@@ -20,7 +20,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 from tests import harness as H  # noqa: E402
-from tests.ref_frames import dataset_for, oracle_cfg  # noqa: E402
+from tests.ref_frames import dataset_for, digest, oracle_cfg, pixel_sample, sample_difference  # noqa: E402
 from oracle import ref_binding as R  # noqa: E402
 from vulkan_renderer_b200 import api  # noqa: E402
 
@@ -183,8 +183,11 @@ def random_config(rng):
 	return cfg
 
 
-def run(frames, seed, width=48, height=32, max_samples=8, with_reference=True, verbose=True, only=None, wild=False, any_config=False):
-	"""Returns (mismatches, compared): dicts with the keys "reference vs oracle" and "device code vs oracle"."""
+def run(frames, seed, width=48, height=32, max_samples=8, with_reference=True, verbose=True, only=None, wild=False, any_config=False, reference_digests=None, record=None):
+	"""Returns (mismatches, compared): dicts with the keys "reference vs oracle" and "device code vs oracle".
+	reference_digests: {frame index (str): {"inputs_sha256", "rgba_sha256", "rgba_sample"}} of the reference shader's frames for these arguments (tests/golden/ref_fuzz.json,
+	written by tools/make_ref_golden.py); the oracle's frames are compared with them instead of running the reference shader. record: a dict that the
+	live reference arm fills with those digests."""
 	import __graft_entry__
 	dev = C.CDLL(__graft_entry__.build_device_on_host())
 	rng = np.random.default_rng(seed)
@@ -218,8 +221,19 @@ def run(frames, seed, width=48, height=32, max_samples=8, with_reference=True, v
 			print("MISMATCH device G-buffer code vs oracle: frame %d seed %d %s %dx%d" % (f, seed, cfg["name"], width, height), flush=True)
 		out, _ = oi.shade(oracle_cfg(cfg, width, height), constants, gb)
 		lit += int((out[..., :3].sum(-1) > 0).any()); pink += int(((out[..., 1] == 0) & (out[..., 0] > 0) & (out[..., 2] > 0)).any())
-		if with_reference:
+		if with_reference and reference_digests is not None:
+			stored = reference_digests[str(f)]
+			compared["reference vs oracle"] += 1
+			if digest(constants, vis) != stored["inputs_sha256"]:
+				mismatches["reference vs oracle"] += 1
+				print("MISMATCH reference vs oracle: frame %d seed %d %s %dx%d: the inputs (constant block, visibility) differ from the stored frame's" % (f, seed, cfg["name"], width, height), flush=True)
+			elif digest(out) != stored["rgba_sha256"]:
+				mismatches["reference vs oracle"] += 1
+				print("MISMATCH reference vs oracle: frame %d seed %d %s %dx%d, sampled pixels: %s" % (f, seed, cfg["name"], width, height, sample_difference(out, stored["rgba_sample"])), flush=True)
+		elif with_reference:
 			ref = R.shade(cfg["entry"], width, height, cfg, constants, vis, oi.vks, oi.material_params, oi.noise, oi.ltc0, oi.ltc1, oi.shadow_tris, textures=oi.textures, light_textures=oi.light_textures)
+			if record is not None:
+				record[str(f)] = {"inputs_sha256": digest(constants, vis), "rgba_sha256": digest(ref), "rgba_sample": pixel_sample(ref)}
 			compared["reference vs oracle"] += 1
 			if not np.array_equal(out.view(np.uint32), ref.view(np.uint32)):
 				mismatches["reference vs oracle"] += 1
